@@ -11,6 +11,7 @@ configuration (configs[1], the one the roofline kernel is quoted on) is measured
     python bench.py --gpus 1 --steps 20 --warmup 3
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference        # CPU arm: the oracle port of the Rust reference on the host cores
+    python bench.py --dump-outputs DIR      # also keep what the last timed step decoded, to compare two builds
 
 JSON keys beyond the base contract: roofline (dominant kernel, CUDA-event timed on the decoder's stream), cpu_baseline
 (oracle on the host cores), e2e (pageable host buffers through the C-ABI batch call), e2e_apt_decode (one apt_decode()
@@ -58,7 +59,13 @@ def parse_args():
     ap.add_argument("--seed-base", type=int, default=0,
                     help="first recording seed of rank 0 (rank r uses seed-base + 4r ...); 12 puts the tied recording, seed 15, on one GPU")
     ap.add_argument("--no-extras", action="store_true", help="skip the single-recording and other-rate measurements")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned to each decoder's caller as DIR/*.npy "
+                         "(image lines, sync positions), at most 64 MB in all; the same arguments give the same inputs")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def measured_peaks():
@@ -267,6 +274,29 @@ def nerr(got, ref):
     return float(np.max(np.abs(got.astype(np.float64) - ref.astype(np.float64)))) / (scale or 1.0)
 
 
+DUMP_BYTES = 64_000_000     # --dump-outputs: every file of every rank together
+LINE = 2080                 # values per decoded image line
+
+
+def dump_arrays(decs, out_devs, produced, world):
+    """What decoder k handed its caller in the last step: `sync_k` (its sync positions) and `rows_k` (its image lines).
+    Every line while all of them fit this rank's share of DUMP_BYTES; otherwise the same seeded sample of lines from
+    each recording, ascending, with their indices in `lines_k`.  Integers are stored as float64 (exact below 2**53)."""
+    import torch
+    arrays = {f"sync_{k:03d}": d.last_sync().astype(np.float64) for k, d in enumerate(decs)}
+    room = DUMP_BYTES // world - sum(a.nbytes for a in arrays.values()) - 3 * 128 * len(decs)   # 128: one .npy header
+    share = max(room, 0) // ((4 * LINE + 8) * len(decs))                                        # lines per recording
+    for k, out in enumerate(out_devs):
+        lines = int(produced[k]) // LINE
+        idx = np.arange(lines)
+        if lines > share:
+            idx = np.sort(np.random.default_rng(0).choice(lines, share, replace=False))
+        sel = torch.from_numpy(idx).to(out.device)
+        arrays[f"rows_{k:03d}"] = out[: lines * LINE].view(lines, LINE).index_select(0, sel).cpu().numpy()
+        arrays[f"lines_{k:03d}"] = idx.astype(np.float64)
+    return arrays
+
+
 def run_b200(args, rank, local_rank, world):
     import torch
     import noaa_apt_b200 as na
@@ -367,6 +397,7 @@ def run_b200(args, rank, local_rank, world):
     ms_step = ms_total / K
     sync_dev = [decs[k].last_sync() for k in range(n_seeds)]
     rows_dev = [out_devs[k][: produced[k]].cpu().numpy() for k in range(n_seeds)]
+    dumped = dump_arrays(decs, out_devs, produced, world) if args.dump_outputs else None   # before later legs reuse decoder 0
 
     # ---- end-to-end arm ("e2e"): the reference-facing batch call on ordinary PAGEABLE host buffers, H2D + D2H inside ----
     outs = [np.zeros(bound, dtype=np.float32) for _ in range(B)]        # zeros: the pages exist before the timed region
@@ -578,6 +609,11 @@ def run_b200(args, rank, local_rank, world):
             "clocks": clocks,
         }
         print(json.dumps(line), flush=True)
+    if dumped is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        prefix = "" if world == 1 else f"rank{rank}_"
+        for name, a in dumped.items():
+            np.save(os.path.join(args.dump_outputs, prefix + name + ".npy"), a)
     for d in decs:
         d.close()
     if dist_on:

@@ -6,6 +6,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -55,3 +56,33 @@ def test_gpu_arm_fails_loudly_without_a_device():
     r = _run(["--steps", "1", "--warmup", "3", "--seconds", "20", "--no-cpu-baseline"])
     assert r.returncode != 0                                  # no CPU fallback for the product path
     assert not any(l.strip().startswith("{") for l in r.stdout.splitlines())
+
+
+def test_dump_arrays_keeps_every_line_or_one_seeded_sample_within_the_budget():
+    import torch
+    import bench
+
+    class Dec:
+        def __init__(self, k):
+            self.k = k
+
+        def last_sync(self):
+            return np.arange(self.k, self.k + 40, dtype=np.uint64) * 6240
+
+    outs = [torch.arange(k, k + 300 * bench.LINE, dtype=torch.float32) for k in range(3)]
+    produced = [300 * bench.LINE] * 3
+    decs = [Dec(k) for k in range(3)]
+    full = bench.dump_arrays(decs, outs, produced, world=1)
+    assert np.array_equal(full["lines_001"], np.arange(300))
+    assert np.array_equal(full["rows_001"], outs[1].numpy().reshape(300, bench.LINE))
+    assert np.array_equal(full["sync_002"], decs[2].last_sync().astype(np.float64))
+    # a world of 500 ranks leaves this rank room for fewer lines than it decoded: a sample, the same on every call
+    part = bench.dump_arrays(decs, outs, produced, world=500)
+    again = bench.dump_arrays(decs, outs, produced, world=500)
+    assert sum(a.nbytes for a in part.values()) <= bench.DUMP_BYTES // 500
+    for k in range(3):
+        idx = part[f"lines_{k:03d}"].astype(np.int64)
+        assert 0 < idx.size < 300 and np.all(np.diff(idx) > 0)
+        assert np.array_equal(idx, again[f"lines_{k:03d}"])
+        assert np.array_equal(part[f"rows_{k:03d}"], outs[k].numpy().reshape(300, bench.LINE)[idx])
+    assert all(a.dtype in (np.float32, np.float64) for a in part.values())

@@ -20,6 +20,8 @@ NVCC_FLAGS = [
     "-Xcompiler", "-fPIC,-ffp-contract=off,-fno-fast-math,-Wall",
     "-cudart", "static",
     "-shared",
+    # compress the sm_100a image (14 -> 3 MB of library); without this nvcc leaves an 8 MB image uncompressed
+    "-Xfatbin", "-compress-all",
 ]
 
 

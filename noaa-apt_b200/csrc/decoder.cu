@@ -370,48 +370,6 @@ static int enqueue_front(apt_decoder *d, const void *in, int format, uint64_t n,
 // Enqueues the whole of decode() on the decoder's stream.  `in` and `rows_out` are device pointers.
 std::atomic<int> g_jobs_in_flight[64];      // per CUDA device: decodes submitted and not yet waited for
 
-// The envelope e (4 N_w bytes, 45 MB for 15 min) is written by the resampler and read by the record and the gather
-// kernels; between those, the resampler's 173 MB input stream pushes most of it out of the 126 MB L2, so e goes to DRAM
-// and comes back (ncu in application order: 273 MB of DRAM traffic per decode against 188 MB algorithmic).  When this is the
-// only decode on the device, e can get a PERSISTING access-policy window on the decoder's stream (everything else the
-// stream touches is treated as streaming): 201 MB per decode, same speed (the kernels that read e are not memory bound).
-// With several decodes in flight the set-aside would only shrink the cache, so the window is dropped then.
-// OPT-IN (APTB200_L2_WINDOW=1): measured on one GPU only; the 4-GPU run that would have validated it next to NCCL and in
-// a multi-device process did not complete, and a device-wide L2 carve-out is not something to switch on unverified.
-static void set_envelope_l2_window(apt_decoder *d, uint64_t nwork, bool alone) {
-    static const bool disabled = getenv("APTB200_L2_WINDOW") == nullptr;
-    static std::atomic<int> setaside[64];              // per device: bytes set aside (0 not tried yet, -1 unsupported)
-    static std::atomic<int> window_max[64];            // per device: largest access-policy window
-    if (disabled || d->device < 0 || d->device >= 64 || !d->d_e) return;
-    int have = setaside[d->device].load(std::memory_order_acquire);
-    if (have == 0) {
-        int max_persist = 0, max_window = 0;
-        cudaDeviceGetAttribute(&max_persist, cudaDevAttrMaxPersistingL2CacheSize, d->device);
-        cudaDeviceGetAttribute(&max_window, cudaDevAttrMaxAccessPolicyWindowSize, d->device);
-        have = -1;
-        if (max_persist > 0 && max_window > 0) {
-            const size_t want = std::min<size_t>(static_cast<size_t>(max_persist), 64u << 20);
-            if (cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, want) == cudaSuccess) have = static_cast<int>(want);
-        }
-        cudaGetLastError();
-        window_max[d->device].store(max_window, std::memory_order_release);
-        setaside[d->device].store(have, std::memory_order_release);
-    }
-    if (have <= 0) return;
-    const uint64_t wmax = static_cast<uint64_t>(window_max[d->device].load(std::memory_order_acquire));
-    const uint64_t bytes = alone ? std::min<uint64_t>(nwork * sizeof(float), wmax) : 0;   // larger than the set-aside: hitRatio < 1
-    if (bytes == d->l2_window_bytes) return;
-    cudaStreamAttrValue v{};
-    v.accessPolicyWindow.base_ptr = d->d_e;
-    v.accessPolicyWindow.num_bytes = static_cast<size_t>(bytes);
-    v.accessPolicyWindow.hitRatio = bytes ? std::min(1.0f, static_cast<float>(have) / static_cast<float>(bytes)) : 0.f;
-    v.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-    v.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
-    if (cudaStreamSetAttribute(d->stream, cudaStreamAttributeAccessPolicyWindow, &v) == cudaSuccess) d->l2_window_bytes = bytes;
-    if (bytes == 0) cudaCtxResetPersistingL2Cache();   // lines that still persist would keep the set-aside from everybody else
-    cudaGetLastError();
-}
-
 int decoder_enqueue(apt_decoder *d, const void *in, int format, uint64_t n, int sync, float *rows_out,
                     const void *host_chunked) {
     const Plan &p = d->plan;
@@ -420,7 +378,6 @@ int decoder_enqueue(apt_decoder *d, const void *in, int format, uint64_t n, int 
     const uint64_t nwork = plan_work_len(p, n);
     d->job_work = nwork;
     d->ev_used = 0;
-    set_envelope_l2_window(d, nwork, c.busy == 0);
 
     if (sync && d->use_records && d->d_ctl) APT_CUDA(cudaMemsetAsync(d->d_ctl, 0, sizeof(SyncCtl), d->stream));
     APT_TRY(enqueue_front(d, in, format, n, nwork, host_chunked));

@@ -85,7 +85,6 @@ struct apt_decoder {
     uint64_t conv_cap = 0;         // samples d_conv holds
     float *d_r = nullptr;          // resampled signal, only for the L == 1 first stage
     float *d_e = nullptr;          // envelope           ("demodulation_result")
-    uint64_t l2_window_bytes = 0;  // bytes of d_e covered by a persisting L2 access-policy window on `stream` (0: none)
     // fused sync stage (kernels_sync2.cuh): f and corr never reach HBM; per-tile records -> roots
     bool use_records = false;      // the fused stage serves this plan (standard / fast / slow profiles)
     aptb200::u32 tile_w = 0, max_tiles = 0, pool_cap = 0, pool_region = 0;   // pool_region: records of a tile's own pool region

@@ -134,8 +134,6 @@ void CopyPool::copy(void *dst, const void *src, size_t bytes) {
 
 HostStager::HostStager(int device, size_t chunk_bytes, int ring, int threads)
     : device_(device), chunk_(chunk_bytes), pool_(threads, device) {
-    if (const char *e = getenv("APTB200_COPY_CHUNK_MB")) chunk_ = std::max<size_t>(1, static_cast<size_t>(atoi(e))) << 20;
-    if (const char *e = getenv("APTB200_COPY_RING")) ring = std::max(2, atoi(e));
     ring_.assign(ring, nullptr);
     ev_.assign(ring, nullptr);
     used_.assign(ring, false);

@@ -123,16 +123,10 @@ template <bool ENVELOPE>
 __global__ void __launch_bounds__(32 * (13 + kWsEpilogueWarps + 1), 1)
 k_polyphase_ws(const float *__restrict__ signal, u64 len, const float *__restrict__ tile_taps,
                const u32 *__restrict__ group_xs, TilePlan tp, u64 nout, u64 tile_begin, u64 ntiles, float cosphi2,
-               float sinphi, float *__restrict__ out, unsigned long long *__restrict__ prof) {
+               float sinphi, float *__restrict__ out) {
     // tiles [tile_begin, ntiles) are computed; `signal` may be a biased pointer into a chunk buffer (signal + x is
     // valid for every sample x those tiles touch), `len` is always the length of the whole signal
     constexpr int Q = kTileQ, KS = kTileKS, QT = kTileQT, E = kWsEpilogueWarps;
-    // optional phase timing (APTB200_TILE_PROFILE): cycles summed over the tiles of CTA 0, lane 0 of one warp per role
-    const bool profiling = prof != nullptr && blockIdx.x == 0 && (threadIdx.x & 31) == 0;
-    const long long t_kernel0 = clock64();
-    long long pt[4] = {0, 0, 0, 0}, t_mark = 0;
-#define PROF_MARK() do { if (profiling) t_mark = clock64(); } while (0)
-#define PROF_ADD(i) do { if (profiling) { const long long now__ = clock64(); pt[i] += now__ - t_mark; t_mark = now__; } } while (0)
     extern __shared__ __align__(128) unsigned char smem_raw[];
     // layout: [8 mbarriers + halo, 128 B][taps][stage 0: rows, halo row][stage 1][planes]
     unsigned long long *bars = reinterpret_cast<unsigned long long *>(smem_raw);
@@ -189,12 +183,8 @@ k_polyphase_ws(const float *__restrict__ signal, u64 len, const float *__restric
             const u64 x_end = x_base + static_cast<u64>(QT - 1) * tp.p_in + tp.row_len;
             const bool want_halo = ENVELOPE && tile > 0;
             const u64 x_halo = x_base - tp.p_in + w0_last;                   // meaningful only when tile > 0
-            PROF_MARK();
             mbar_wait(empty_rows + st, ((n >> 1) & 1) ^ 1);                 // stage free (first use passes)
-            PROF_ADD(0);
-            if (tp.debug == 2) {
-                if (lane == 0) mbar_arrive(full_rows + st);
-            } else if (aligned16) {
+            if (aligned16) {
                 // One bulk copy per row pair (rows 2i, 2i+1 overlap in the signal).  The part of a pair that
                 // exists (a multiple of 4 floats) comes by TMA; the rest -- the last <4 samples and everything
                 // past the end of the signal, which reads as zero (signal.get(x) == None, dsp.rs:257) -- by this
@@ -258,9 +248,7 @@ k_polyphase_ws(const float *__restrict__ signal, u64 len, const float *__restric
                 __syncwarp();
                 if (lane == 0) mbar_arrive(full_rows + st);
             }
-            PROF_ADD(1);
         }
-        if (profiling) { prof[0] = pt[0]; prof[1] = pt[1]; }
     } else if (is_compute) {
         // ======================================= compute ========================================
         const u32 ks = lane >> 3, ql = lane & 7;
@@ -281,43 +269,39 @@ k_polyphase_ws(const float *__restrict__ signal, u64 len, const float *__restric
         for (u64 tile = tile_begin + blockIdx.x; tile < ntiles; tile += gridDim.x, ++n) {
             const u32 st = n & 1;
             const float *rows = s_stage0 + st * tp.stage_floats;
-            PROF_MARK();
             mbar_wait(full_rows + st, (n >> 1) & 1);
-            PROF_ADD(0);
             f32x2 acc_a[2][Q], acc_b[2][Q];
 #pragma unroll
             for (int p = 0; p < 2; ++p)
 #pragma unroll
                 for (int j = 0; j < Q; ++j) acc_a[p][j] = acc_b[p][j] = 0ull;
-            if (tp.debug != 1 && tp.debug < 5) {
-                u32 tap_addr = tap_base;
-                u32 row_addr = smem_u32(rows) + row_off;
-                u32 it = 0;
-                for (; it < it_b_begin; ++it) {                        // half A only
-                    float4 s[Q];
+            u32 tap_addr = tap_base;
+            u32 row_addr = smem_u32(rows) + row_off;
+            u32 it = 0;
+            for (; it < it_b_begin; ++it) {                            // half A only
+                float4 s[Q];
 #pragma unroll
-                    for (int j = 0; j < Q; ++j) s[j] = lds128(row_addr + j * row_step8);
-                    half_fma2(acc_a, tap_addr, s);
-                    row_addr += KS * 16;
-                    tap_addr += rec_bytes;
-                }
-                for (; it < it_a_end; ++it) {                          // both halves
-                    float4 s[Q];
+                for (int j = 0; j < Q; ++j) s[j] = lds128(row_addr + j * row_step8);
+                half_fma2(acc_a, tap_addr, s);
+                row_addr += KS * 16;
+                tap_addr += rec_bytes;
+            }
+            for (; it < it_a_end; ++it) {                              // both halves
+                float4 s[Q];
 #pragma unroll
-                    for (int j = 0; j < Q; ++j) s[j] = lds128(row_addr + j * row_step8);
-                    half_fma2(acc_a, tap_addr, s);
-                    half_fma2(acc_b, tap_addr + 64, s);
-                    row_addr += KS * 16;
-                    tap_addr += rec_bytes;
-                }
-                for (; it < tp.iters; ++it) {                          // half B only
-                    float4 s[Q];
+                for (int j = 0; j < Q; ++j) s[j] = lds128(row_addr + j * row_step8);
+                half_fma2(acc_a, tap_addr, s);
+                half_fma2(acc_b, tap_addr + 64, s);
+                row_addr += KS * 16;
+                tap_addr += rec_bytes;
+            }
+            for (; it < tp.iters; ++it) {                              // half B only
+                float4 s[Q];
 #pragma unroll
-                    for (int j = 0; j < Q; ++j) s[j] = lds128(row_addr + j * row_step8);
-                    half_fma2(acc_b, tap_addr + 64, s);
-                    row_addr += KS * 16;
-                    tap_addr += rec_bytes;
-                }
+                for (int j = 0; j < Q; ++j) s[j] = lds128(row_addr + j * row_step8);
+                half_fma2(acc_b, tap_addr + 64, s);
+                row_addr += KS * 16;
+                tap_addr += rec_bytes;
             }
             // r[K0 - 1]: the last output of the last group, applied to the halo row
             float halo = 0.f;
@@ -336,10 +320,8 @@ k_polyphase_ws(const float *__restrict__ signal, u64 len, const float *__restric
             }
             __syncwarp();
             if (lane == 0) mbar_arrive(empty_rows + st);           // this warp is done with the stage
-            PROF_ADD(1);
             // hand the partial sums to the epilogue warps
             mbar_wait(empty_p, (n & 1) ^ 1);
-            PROF_ADD(2);
 #pragma unroll
             for (int j = 0; j < Q; ++j) {
                 float4 va, vb;
@@ -354,9 +336,7 @@ k_polyphase_ws(const float *__restrict__ signal, u64 len, const float *__restric
             if (ENVELOPE && warp == G - 1 && lane == 0) *s_halo = halo;
             __syncwarp();
             if (lane == 0) mbar_arrive(full_p);
-            PROF_ADD(3);
         }
-        if (profiling && warp == 0) { prof[2] = pt[0]; prof[3] = pt[1]; prof[4] = pt[2]; prof[5] = pt[3]; }
     } else {
         // ======================================= epilogue =======================================
         const u32 e = warp - G - (warp > prod_warp ? 1 : 0);   // epilogue warps: every remaining warp, in order
@@ -370,9 +350,7 @@ k_polyphase_ws(const float *__restrict__ signal, u64 len, const float *__restric
             const u64 k_base = tile * tile_out;
             const bool full_tile = k_base + tile_out <= nout && out_aligned;
             float *out_tile = out + k_base;
-            PROF_MARK();
             mbar_wait(full_p, n & 1);
-            PROF_ADD(0);
             // two cells per lane and pass (independent chains -> ILP); cells are 4 consecutive outputs
             for (u32 v0 = e * 32 + lane; v0 < nvec; v0 += 2 * E * 32) {
 #pragma unroll
@@ -413,18 +391,8 @@ k_polyphase_ws(const float *__restrict__ signal, u64 len, const float *__restric
             }
             __syncwarp();
             if (lane == 0) mbar_arrive(empty_p);
-            PROF_ADD(1);
-        }
-        if (profiling && e == 0) { prof[6] = pt[0]; prof[7] = pt[1]; prof[8] = n; }
-        if (prof != nullptr && e == 0 && lane == 0) {   // per-CTA wall time of the whole kernel body + SM id
-            u32 smid;
-            asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
-            prof[16 + 2 * blockIdx.x] = clock64() - t_kernel0;
-            prof[17 + 2 * blockIdx.x] = smid;
         }
     }
-#undef PROF_MARK
-#undef PROF_ADD
 }
 
 }  // namespace aptb200

@@ -533,7 +533,6 @@ k_pick_j0(u64 ncorr, u32 row, u32 dist, const RootIndex ri, u32 *__restrict__ po
         sc.cand_s[c] = s;
         sc.cand_peak[c] = peak;
         sc.ja[c] = nxt;
-        if (sc.idx) sc.idx[c] = 0;      // image flags of the compressed walk (k_pick_e8 sets them)
     }
     if (c == 0) {
         // the first start, from the seed (decode.rs:208-209)
@@ -638,137 +637,6 @@ k_pick_cluster(u64 ncorr, u64 nwork, u32 row, u32 dist, const RootIndex ri, u32 
     u32 cnt = 0;
     for (u32 i = tid; i + 1 < npeaks; i += T)
         if (static_cast<u64>(__ldcg(positions + i)) + row < nwork) ++cnt;
-    const u32 total_rows = block_scan_inclusive_1024(cnt, s_tmp);
-    if (tid == T - 1) {
-        result->n_peaks = npeaks;
-        result->n_rows = total_rows;
-        result->status = npeaks < 5 ? 3u : 0u;
-        result->n_roots = nroots;
-    }
-}
-
-// ---------------------------------------------------------------------------------------------
-// Compressed orbit walk (the default for recordings up to a few hours): orbits of the monotone map F merge quickly, so
-// the image of E = F^R (R = 8 steps) over ALL ~62 k candidate starts is only a few hundred nodes -- and once the orbit
-// has made one E-step it never leaves that image.  So:
-//   k_pick_j0  (whole GPU) : J0 = F for every node                                (chains of dependent root-list searches)
-//   k_pick_e8  (whole GPU) : E[c] = J0^8[c], flag[E[c]] = 1                       (8 dependent L2 loads per node)
-//   k_pick_final (ONE CTA) : compact the flagged nodes (K of them), E restricted to them in SHARED memory, pointer doubling
-//                            over K nodes with __syncthreads only (orbit in steps of 8), expansion of every 8-step by a walk
-//                            through J0, events -> positions, counts.
-// No grid barrier, no cluster: ~20 us instead of 39 us (11 grid barriers) for a 15-minute recording, and the single CTA
-// leaves the GPU to the other streams of a batch.  Falls back to the one-thread walk when K exceeds the shared-memory table.
-// ---------------------------------------------------------------------------------------------
-constexpr u32 kPickR = 8;
-constexpr u32 kPickKMax = 12288;       // compact nodes: two u32 tables of dynamic shared memory (96 KB)
-constexpr u32 kPickEMax = 6144;        // E-steps of the orbit kept in shared memory (rows / 8 + 2: ~13 h of recording)
-
-__global__ void __launch_bounds__(256)
-k_pick_e8(u64 ncorr, u32 row, const RootIndex ri, u32 max_positions, const SyncResult *__restrict__ result, PickScratch sc) {
-    if (result->status == kSyncRedo) return;
-    const u32 nroots = __ldcg(ri.nroots);
-    const u32 nr = static_cast<u32>((ncorr + row - 1) / row);
-    const u32 ncand = nr + nroots;
-    if (ncand + 1 > sc.cap || nr + 1 > max_positions) return;
-    const u32 c = blockIdx.x * blockDim.x + threadIdx.x;
-    if (c > ncand) return;
-    u32 v = c;
-#pragma unroll
-    for (u32 t = 0; t < kPickR; ++t) v = __ldcg(sc.ja + v);      // END is absorbing
-    sc.jb[c] = v;
-    sc.idx[v] = 1u;                                              // zeroed by k_pick_j0
-}
-
-__global__ void __launch_bounds__(1024, 1)
-k_pick_final(u64 ncorr, u64 nwork, u32 row, u32 dist, const RootIndex ri, u32 *__restrict__ positions, u32 max_positions,
-             SyncResult *__restrict__ result, PickScratch sc) {
-    extern __shared__ u32 pf_smem[];            // [2][kPickKMax] tables, [kPickKMax] node of a compact id, [kPickEMax] orbit in E-steps
-    __shared__ u32 s_tmp[32];
-    __shared__ u32 s_misc[4];
-    u32 *tab0 = pf_smem, *tab1 = pf_smem + kPickKMax, *node_of = pf_smem + 2 * kPickKMax, *orbe = pf_smem + 3 * kPickKMax;
-    const u32 tid = threadIdx.x;
-    constexpr u32 T = 1024;
-    if (result->status == kSyncRedo) return;
-    const u32 nroots = __ldcg(ri.nroots);
-    const u32 nr = static_cast<u32>((ncorr + row - 1) / row);
-    const u32 ncand = nr + nroots;
-    const u32 END = ncand;
-    const u32 max_events = min(nr + 1, max_positions);   // every event lands in a new row
-    const u32 n_e = (max_events + kPickR - 1) / kPickR + 1;   // E-steps that can hold events
-    bool fallback = ncand + 1 > sc.cap || nr + 1 > max_positions || n_e > kPickEMax;
-    // ---- compact ids of the flagged nodes: exclusive scan of the flags (each thread a contiguous chunk) ----
-    u32 K = 0;
-    if (!fallback) {
-        const u32 per = (ncand + 1 + T - 1) / T;
-        const u32 c0 = min(tid * per, ncand + 1), c1 = min(c0 + per, ncand + 1);
-        u32 local = 0;
-        for (u32 c = c0; c < c1; ++c) local += __ldcg(sc.idx + c);
-        const u32 incl = block_scan_inclusive_1024(local, s_tmp);
-        if (tid == T - 1) s_misc[0] = incl;
-        __syncthreads();
-        K = s_misc[0];
-        if (K > kPickKMax) {
-            fallback = true;
-        } else {
-            u32 id = incl - local;
-            for (u32 c = c0; c < c1; ++c)
-                if (__ldcg(sc.idx + c)) { sc.idx[c] = id; node_of[id] = c; ++id; }
-        }
-    }
-    if (fallback) {
-        if (tid == 0) {
-            pick_sequential(ncorr, nwork, row, dist, ri, positions, max_positions, result);
-            result->n_roots = nroots;
-        }
-        return;
-    }
-    __syncthreads();
-    // E restricted to the image, in compact ids
-    for (u32 k = tid; k < K; k += T) tab0[k] = __ldcg(sc.idx + __ldcg(sc.jb + node_of[k]));
-    // the orbit in E-steps: c_0 = the start node itself (raw id), c_i (i >= 1) compact
-    const u32 s0 = __ldcg(sc.orbit + 0);
-    if (tid == 0) orbe[1] = __ldcg(sc.idx + __ldcg(sc.jb + s0));
-    __syncthreads();
-    u32 *tc = tab0, *tn = tab1;
-    for (u32 span = 1; span + 1 < n_e; span <<= 1) {
-        for (u32 n = tid; n < span && 1 + n + span < n_e; n += T) orbe[1 + n + span] = tc[orbe[1 + n]];
-        if ((span << 1) + 1 < n_e)
-            for (u32 k = tid; k < K; k += T) tn[k] = tc[tc[k]];
-        __syncthreads();
-        u32 *t2 = tc; tc = tn; tn = t2;
-    }
-    // ---- expansion: the kPickR nodes of every E-step by a walk through J0 ----
-    for (u32 i = tid; i < n_e; i += T) {
-        u32 v = i == 0 ? s0 : node_of[orbe[i]];
-#pragma unroll
-        for (u32 t = 0; t < kPickR; ++t) {
-            const u32 n = i * kPickR + t;
-            if (n < max_events) sc.orbit[n] = v;
-            v = __ldcg(sc.ja + v);
-        }
-    }
-    __syncthreads();
-    // ---- events -> positions (decode.rs:241-253); END is absorbing so events are a prefix of orbit[] ----
-    for (u32 n = tid; n < max_events; n += T) {
-        const u32 v = sc.orbit[n];
-        if (v == END) continue;
-        const u32 s = __ldcg(sc.cand_s + v);
-        const u32 target = s / row;
-        const u32 prev = n == 0 ? 1u : __ldcg(sc.cand_s + sc.orbit[n - 1]) / row;
-        for (u32 j = prev; j + 1 < target; ++j) positions[j] = s;      // duplicates pushed by the `while`
-        positions[target - 1] = __ldcg(sc.cand_peak + v);
-    }
-    __syncthreads();
-    u32 my_events = 0;
-    for (u32 n = tid; n < max_events; n += T) my_events += sc.orbit[n] != END;
-    const u32 events = block_scan_inclusive_1024(my_events, s_tmp);
-    if (tid == T - 1) s_misc[2] = events;
-    __syncthreads();
-    const u32 nev = s_misc[2];
-    const u32 npeaks = nev == 0 ? 1u : __ldcg(sc.cand_s + sc.orbit[nev - 1]) / row;
-    u32 cnt = 0;
-    for (u32 i = tid; i + 1 < npeaks; i += T)
-        if (static_cast<u64>(positions[i]) + row < nwork) ++cnt;
     const u32 total_rows = block_scan_inclusive_1024(cnt, s_tmp);
     if (tid == T - 1) {
         result->n_peaks = npeaks;

@@ -29,20 +29,16 @@
 
 namespace aptb200 {
 
-// TB = rows of 32 low-passed samples per tile: 64 (two rounds of a warp per phase, 6.7 % halo, 19.3 KB of shared memory per
-// warp -> 11 warps per SM) or 32 (one round, 14 % halo, 10 KB -> 20 warps per SM).
+constexpr int kRecTB = 64;                       // rows of 32 low-passed samples per tile (two rounds of a warp per phase)
 constexpr int kRecRowPitch = 36;                 // floats per shared-memory row of 32 (+4: 16-byte accesses of 8
                                                  // consecutive rows hit 8 distinct bank groups)
 constexpr int kRecShift = 3;                     // box-sum row r lives in physical row r + 3 (aliases dead e rows)
-__host__ __device__ constexpr int rec_smem_floats(int tb) { return (tb + kRecShift) * kRecRowPitch; }
-// NBUF = 2: the next tile's samples are in flight while the current tile is worked on; NBUF = 1: half the shared memory,
-// so nearly twice the warps per SM (the register file becomes the limit), each waiting for its own tile's samples.
-__host__ __device__ constexpr int rec_ctas_per_sm(int tb, int nt, int nbuf = 2) {
-    return nbuf == 2 ? (tb >= 64 ? 11 : (nt > 43 ? 12 : 20)) : (nt > 43 ? 12 : nt > 37 ? 16 : 20);
-}
+constexpr int kRecSmemFloats = (kRecTB + kRecShift) * kRecRowPitch;   // shared memory of one warp (9.4 KB)
+// one warp per CTA, each waiting for its own tile's samples: the register file limits the warps per SM
+__host__ __device__ constexpr int rec_ctas_per_sm(int nt) { return nt > 43 ? 12 : nt > 37 ? 16 : 20; }
 
-__host__ __device__ constexpr int rec_tile_outputs(int pw, int tb) {   // W: correlation outputs per tile (multiple of 32)
-    return (32 * tb - 18 * 2 * pw - (2 * pw - 1)) / 32 * 32;
+__host__ __device__ constexpr int rec_tile_outputs(int pw) {   // W: correlation outputs per tile (multiple of 32)
+    return (32 * kRecTB - 18 * 2 * pw - (2 * pw - 1)) / 32 * 32;
 }
 
 __device__ __forceinline__ float warp_max_all(float v) {
@@ -81,8 +77,8 @@ __device__ __forceinline__ u32 warp_excl_sum(u32 v, u32 lane, u32 &total) {
 }
 
 // ------------------------------------------------------------------------------------------------------------------
-// k_lowpass_records.  One warp = one tile at a time (tiles are drawn from a global ticket): positions
-// [i0, i0 + W), i0 = tile * W.  Shared memory per warp: (TB + 3) rows of 36 floats.
+// k_lowpass_records.  One CTA = one warp = one tile at a time: positions [i0, i0 + W), i0 = tile * W.  Shared memory:
+// (TB + 3) rows of 36 floats.
 //   stage   : e[i0 - EOFF, i0 + 32*TB) -> rows (logical index m <-> e[i0 - EOFF + m]); samples with index < 1 or >= n
 //             are zero (dsp.rs:399: signal[0] is never read)
 //   phase 1 : lane = one row of 32 consecutive outputs f[i0 + 32r ..]: the 32+EOFF window in registers as packed pairs,
@@ -103,20 +99,16 @@ __device__ __forceinline__ void cp_async8(Rec *dst, const Rec *src) {
 __device__ __forceinline__ void cp_async_commit_group() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_group 0;" ::: "memory"); }
 
-// NW = 1 (what is instantiated): every warp is its own CTA.  NW > 1: the NW warps of a CTA take NW consecutive tiles and
-// meet at a CTA barrier before every phase, so that they share the fetched instruction lines (the kernel is ~3900
-// straight-line instructions per tile, 46 KB of code).  Measured at NW = 4 / 8 / 10 / 16 / 20: 49.5 / 49.5 / 55.6 / 65.9 /
-// 59.7 us against 47.6 us for NW = 1 -- instruction supply is not what bounds the kernel; kept as a template parameter only.
-template <int NT, int PW, int TB, int NBUF = 2, int NW = 1>
-__global__ void __launch_bounds__(32 * NW, rec_ctas_per_sm(TB, NT, NBUF) / NW > 0 ? rec_ctas_per_sm(TB, NT, NBUF) / NW : 1)
+template <int NT, int PW>
+__global__ void __launch_bounds__(32, rec_ctas_per_sm(NT))
 k_lowpass_records(const float *__restrict__ e, u64 n, u64 ncorr, const __grid_constant__ LpTaps taps, SyncCtl *__restrict__ ctl,
                   TileDesc *__restrict__ desc, Rec *__restrict__ pool, u32 pool_cap, u32 region, u32 ntiles) {
     constexpr int BOX = 2 * PW;
     constexpr int LOOK = 18 * BOX;
-    constexpr int W = rec_tile_outputs(PW, TB);
+    constexpr int TB = kRecTB;
+    constexpr int W = rec_tile_outputs(PW);
     constexpr int NI = W / 32;                              // correlation items (rows of 32 outputs) per tile
     constexpr int RD = (NI + 31) / 32;                      // rounds of the correlation phase
-    constexpr int kRecSmemFloats = rec_smem_floats(TB);
     static_assert(TB % 32 == 0 && NI >= 1 && RD <= 2, "one or two rounds of correlation items");
     static_assert(NT % 2 == 1, "odd tap counts only (Kaiser design, filters.rs:79)");
     constexpr int EOFF = (NT - 1 + 3) / 4 * 4;
@@ -127,21 +119,20 @@ k_lowpass_records(const float *__restrict__ e, u64 n, u64 ncorr, const __grid_co
     static_assert(EOFF - (NT - 1) >= 0 && EOFF + 31 + 1 < WN + 1, "window of a row");
     constexpr int PITCH = kRecRowPitch;
 
-    constexpr bool LOCK = NW > 1;
     extern __shared__ __align__(16) float rec_smem[];
-    const u32 warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    float *sbuf = rec_smem + warp * (NBUF * kRecSmemFloats);   // NBUF = 2: the tile in work, the next tile's samples in flight
+    float *const s = rec_smem;
+    const u32 lane = threadIdx.x & 31;
 
-    // e[i0 - EOFF, i0 + 32*TB) -> rows of `buf` (logical index m <-> e[i0 - EOFF + m]); samples with index < 1 or >= n are
+    // e[i0 - EOFF, i0 + 32*TB) -> rows of s (logical index m <-> e[i0 - EOFF + m]); samples with index < 1 or >= n are
     // zero (dsp.rs:399: signal[0] is never read).  Interior tiles: 16-byte cp.async, no registers, no waiting here.
-    auto stage = [&](u32 tile, float *buf) {
+    auto stage = [&](u32 tile) {
         const long long g0 = static_cast<long long>(tile) * W - EOFF;
         if (g0 >= 4 && static_cast<u64>(g0) + LE <= n) {
             const float *src = e + g0;
 #pragma unroll 4
             for (u32 q4 = lane; q4 < LE / 4; q4 += 32) {
                 const u32 m = 4 * q4;
-                cp_async16(buf + (m >> 5) * PITCH + (m & 31), src + m);
+                cp_async16(s + (m >> 5) * PITCH + (m & 31), src + m);
             }
         } else {
             for (u32 q4 = lane; q4 < LE / 4; q4 += 32) {
@@ -152,35 +143,19 @@ k_lowpass_records(const float *__restrict__ e, u64 n, u64 ncorr, const __grid_co
                 v.y = g + 1 >= 1 && static_cast<u64>(g + 1) < n ? __ldg(e + g + 1) : 0.f;
                 v.z = g + 2 >= 1 && static_cast<u64>(g + 2) < n ? __ldg(e + g + 2) : 0.f;
                 v.w = g + 3 >= 1 && static_cast<u64>(g + 3) < n ? __ldg(e + g + 3) : 0.f;
-                *reinterpret_cast<float4 *>(buf + (m >> 5) * PITCH + (m & 31)) = v;
+                *reinterpret_cast<float4 *>(s + (m >> 5) * PITCH + (m & 31)) = v;
             }
         }
         cp_async_commit_group();
     };
-    // Tiles are dealt out statically (every tile costs the same): CTA b takes the tile groups b, b + gridDim.x, ...; a group
-    // is NW consecutive tiles, one per warp.  No tickets: two same-address atomics per tile (ticket + pool cursor, 11.7 k of
-    // them on one cache line) were what kept the first version at ~52 us whatever the occupancy.
-    auto phase_barrier = [&]() {
-        if (LOCK) __syncthreads();
-    };
-    auto tile_of = [&](u32 it) { return (blockIdx.x + it * gridDim.x) * static_cast<u32>(NW) + warp; };
-
-    // A warp whose tile lies beyond the last one (only in the last group, NW > 1) runs along on stale shared memory to keep
-    // the barriers simple; everything it would publish is gated by `active`.
-    u32 tile = tile_of(0);
-    if (tile < ntiles) stage(tile, sbuf);
-    for (u32 it = 0; tile - (LOCK ? warp : 0u) < ntiles; ++it) {
-        const bool active = tile < ntiles;
-        const u32 next = tile_of(it + 1);
-        phase_barrier();
-        float *s = sbuf + (NBUF == 2 ? (it & 1) * kRecSmemFloats : 0);
-        if (NBUF == 2) {
-            if (next < ntiles) stage(next, sbuf + ((it + 1) & 1) * kRecSmemFloats);
-            // the current tile's samples: everything but the group just committed
-            if (next < ntiles) asm volatile("cp.async.wait_group 1;" ::: "memory"); else cp_async_wait_all();
-        } else {
-            cp_async_wait_all();
-        }
+    // Tiles are dealt out statically (every tile costs the same): CTA b takes the tiles b, b + gridDim.x, ...  No tickets:
+    // two same-address atomics per tile (ticket + pool cursor, 11.7 k of them on one cache line) were what kept the first
+    // version at ~52 us whatever the occupancy.
+    u32 tile = blockIdx.x;
+    if (tile < ntiles) stage(tile);
+    for (u32 it = 0; tile < ntiles; ++it) {
+        const u32 next = blockIdx.x + (it + 1) * gridDim.x;
+        cp_async_wait_all();
         __syncwarp();
         const u64 i0 = static_cast<u64>(tile) * W;
 
@@ -190,7 +165,6 @@ k_lowpass_records(const float *__restrict__ e, u64 n, u64 ncorr, const __grid_co
         for (int k = 0; k < BOX - 1; ++k) carry[k] = 0.f;
 #pragma unroll 1
         for (int rb = TB / 32 - 1; rb >= 0; --rb) {
-            phase_barrier();
             const u32 r = 32 * rb + lane;
             const float *row = s + r * PITCH;
             // One window sample x the taps of two neighbouring outputs: FFMA2 R.F32 (broadcast) x UR.pair + R.pair, the form that
@@ -249,7 +223,6 @@ k_lowpass_records(const float *__restrict__ e, u64 n, u64 ncorr, const __grid_co
                 *reinterpret_cast<float4 *>(brow + 4 * k) = make_float4(b[4 * k], b[4 * k + 1], b[4 * k + 2], b[4 * k + 3]);
         }
         __syncwarp();
-        phase_barrier();
 
         // ---- phase 3: correlation, RD rounds of 32 items ----
         float c[RD][32];
@@ -307,7 +280,6 @@ k_lowpass_records(const float *__restrict__ e, u64 n, u64 ncorr, const __grid_co
             mx[rd] = fmaxf(fmaxf(gm[rd][0], gm[rd][1]), fmaxf(gm[rd][2], gm[rd][3]));
         }
 
-        phase_barrier();
         // ---- records: bounds from outside the lane by warp scans, then 8 independent chains of 8 per round ----
         float all[RD], pm[RD], sx[RD];
 #pragma unroll
@@ -367,11 +339,10 @@ k_lowpass_records(const float *__restrict__ e, u64 n, u64 ncorr, const __grid_co
         // space from the shared overflow area behind the regions (region == 0: everything comes from there)
         u32 base = tile * region;
         if (tot_s + tot_p > region) {                       // warp-uniform
-            if (lane == 0 && active) base = ntiles * region + atomicAdd(&ctl->pool_cursor, tot_s + tot_p);
+            if (lane == 0) base = ntiles * region + atomicAdd(&ctl->pool_cursor, tot_s + tot_p);
             base = __shfl_sync(0xffffffffu, base, 0);
         }
-        const bool fits = active && static_cast<u64>(base) + tot_s + tot_p <= pool_cap;
-        phase_barrier();
+        const bool fits = static_cast<u64>(base) + tot_s + tot_p <= pool_cap;
         if (fits) {
             // Every lane writes its own records straight from the registers that hold its 32 correlation values: one
             // predicated 8-byte store per (output, list), 128 per tile, all independent.  (The first version parked the values
@@ -391,13 +362,13 @@ k_lowpass_records(const float *__restrict__ e, u64 n, u64 ncorr, const __grid_co
         float tmax = all[0];
 #pragma unroll
         for (int rd = 1; rd < RD; ++rd) tmax = fmaxf(tmax, all[rd]);
-        if (lane == 0 && active) {
+        if (lane == 0) {
             if (!fits) atomicExch(&ctl->overflow, 1u);
             desc[tile] = TileDesc{base, fits ? tot_s : 0u, fits ? tot_p : 0u, tmax};
         }
         __syncwarp();
         tile = next;
-        if (NBUF == 1 && tile < ntiles) stage(tile, sbuf);
+        if (tile < ntiles) stage(tile);
     }
 }
 

@@ -57,7 +57,6 @@ struct UtGeom {
     u32 header_bytes;         // barriers + halo taps, multiple of 128
     u32 slot_stride;          // floats between slots: slot_floats + the 2*rows+4 exchange words behind each slot
     u32 stream_b;             // float4 index where the second role's tap stream starts
-    u32 debug;
 };
 
 constexpr int CH = static_cast<int>(kUtChunk);   // samples per chunk (one loop iteration)
@@ -81,13 +80,10 @@ __device__ __forceinline__ void ut_load_chunk(const float *p, float (&s)[CH]) {
 
 // Chunks [cb, ce) with pairs [P0, P1) of a role active.  toff: running float4 index into the tap stream (uniform);
 // per (chunk, pair) the stream holds CH/2 float4 = the tap pairs of the chunk's CH samples.
-#ifndef APTB200_UT_STEADY_UNROLL
-#define APTB200_UT_STEADY_UNROLL 1
-#endif
-template <int P0, int P1, int NPR, int Q, int VEC, int MAXV, int UNR = 1>
+template <int P0, int P1, int NPR, int Q, int VEC, int MAXV>
 __device__ __forceinline__ void ut_segment(const UtParams<MAXV> &prm, u32 cb, u32 ce, int &toff, const float *row0,
                                            u32 qstride, f32x2 (&acc)[Q][NPR]) {
-#pragma unroll UNR
+#pragma unroll 1   // unrolled x2 the kernel is slower (code size, DESIGN.md §3.1)
     for (u32 c = cb; c < ce; ++c) {
         float s[Q][CH];
 #pragma unroll
@@ -127,18 +123,7 @@ __device__ __forceinline__ void ut_ramp_down(const UtParams<MAXV> &prm, int &tof
 template <int L, int PB, int NPR, bool LAST, int Q, int VEC, int MAXV, bool ENVELOPE>
 __device__ __forceinline__ void ut_role(const UtParams<MAXV> &prm, const UtGeom &g, int toff, float *slot, u64 *xch_bar,
                                         u64 *staged_bar, u32 parity, u32 role, const float *halo_taps, u64 k0, u64 nout,
-                                        float cosphi2, float inv_sinphi, float *__restrict__ out, u32 lane, bool profiling,
-                                        unsigned long long *prof, long long &pt) {
-#ifdef APTB200_UT_PROFILE
-#define UT_MARK(slot_)                                   \
-    if (profiling) {                                     \
-        const long long now_ = clock64();                \
-        prof[slot_] += now_ - pt;                        \
-        pt = now_;                                       \
-    }
-#else
-#define UT_MARK(slot_)
-#endif
+                                        float cosphi2, float inv_sinphi, float *__restrict__ out, u32 lane) {
     constexpr u32 RB = 32 * Q;
     constexpr int JB = 2 * PB;                                       // first output (phase) of this role
     constexpr int JN = (2 * NPR < L - JB) ? 2 * NPR : L - JB;        // number of real outputs
@@ -149,12 +134,9 @@ __device__ __forceinline__ void ut_role(const UtParams<MAXV> &prm, const UtGeom 
 #pragma unroll
         for (int p = 0; p < NPR; ++p) acc[q][p] = 0ull;
     const float *row0 = slot + g.back + lane * m;
-    if (g.debug != 1) {
-        ut_ramp_up<PB, NPR, Q, VEC, MAXV>(prm, toff, row0, qstride, acc, std::make_integer_sequence<int, NPR - 1>{});
-        ut_segment<0, NPR, NPR, Q, VEC, MAXV, APTB200_UT_STEADY_UNROLL>(prm, prm.cs[PB + NPR - 1], prm.ce[PB], toff, row0, qstride, acc);
-        ut_ramp_down<PB, NPR, Q, VEC, MAXV>(prm, toff, row0, qstride, acc, std::make_integer_sequence<int, NPR - 1>{});
-    }
-    UT_MARK(2)
+    ut_ramp_up<PB, NPR, Q, VEC, MAXV>(prm, toff, row0, qstride, acc, std::make_integer_sequence<int, NPR - 1>{});
+    ut_segment<0, NPR, NPR, Q, VEC, MAXV>(prm, prm.cs[PB + NPR - 1], prm.ce[PB], toff, row0, qstride, acc);
+    ut_ramp_down<PB, NPR, Q, VEC, MAXV>(prm, toff, row0, qstride, acc, std::make_integer_sequence<int, NPR - 1>{});
     // boundary outputs, exchanged through the words behind the slot's samples:
     //   xa[row]     = output JN-1 of the first role (needed by the second role's first output)
     //   xb[row + 1] = output L-1 of the row (needed by the next row's output 0); xb[0] = r[k0-1] (halo)
@@ -180,17 +162,10 @@ __device__ __forceinline__ void ut_role(const UtParams<MAXV> &prm, const UtGeom 
             else xa[q * 32 + lane] = last;
         }
     }
-    UT_MARK(3)
     // both warps are past the FMA loop (nobody reads the samples any more) and have published
     __syncwarp();
     if (lane == 0) mbar_arrive(xch_bar);
-#if defined(APTB200_UT_XCH_SLEEP) && APTB200_UT_XCH_SLEEP > 0
-    // the lighter role (3 of the 7 pairs) waits here for ~a quarter of a block's time: back off between polls so that its
-    // try_wait loop (55 iterations x 4 instructions per block in the first capture) does not eat issue slots
-    while (!mbar_try_wait(xch_bar, parity)) __nanosleep(APTB200_UT_XCH_SLEEP);
-#else
     mbar_wait(xch_bar, parity);
-#endif
 #pragma unroll
     for (int q = 0; q < Q; ++q) {
         float r[2 * NPR];
@@ -212,24 +187,11 @@ __device__ __forceinline__ void ut_role(const UtParams<MAXV> &prm, const UtGeom 
     }
     __syncwarp();
     if (lane == 0) mbar_arrive(staged_bar);
-#ifdef APTB200_UT_ROLE1_STORES
-    // experiment: the lighter role (3 of the 7 pairs) stores the whole block, the heavier one moves on to its next ticket
-    if (!LAST) return;
     mbar_wait(staged_bar, parity);
-    UT_MARK(4)
-    constexpr u32 nvec = RB * L / 4;
-#pragma unroll
-    for (u32 vi = 0; vi < (nvec + 31) / 32; ++vi) {
-        const u32 v = lane + 32 * vi;
-        (void)role;
-#else
-    mbar_wait(staged_bar, parity);
-    UT_MARK(4)
     constexpr u32 nvec = RB * L / 4;                                   // RB*L is a multiple of 4
 #pragma unroll
     for (u32 vi = 0; vi < (nvec + 63) / 64; ++vi) {
         const u32 v = lane + 32 * (2 * vi + role);
-#endif
         const u64 k = k0 + 4 * v;
         if (v >= nvec || k >= nout) break;
         float4 val = *reinterpret_cast<const float4 *>(slot + 4 * v);
@@ -242,14 +204,13 @@ __device__ __forceinline__ void ut_role(const UtParams<MAXV> &prm, const UtGeom 
             if (k + 2 < nout) out[k + 2] = val.z;
         }
     }
-#undef UT_MARK
 }
 
 template <int L, int Q, int VEC, int MAXV, bool ENVELOPE>
-__global__ void __launch_bounds__(Q >= 4 ? 512 : 800, 1)
+__global__ void __launch_bounds__(800, 1)
 k_polyphase_ut(const __grid_constant__ UtParams<MAXV> prm, const float *__restrict__ signal, u64 len,
                const float *__restrict__ h, const UtGeom g, u64 nout, u64 blk_begin, u64 blk_end, float cosphi2,
-               float inv_sinphi, float *__restrict__ out, unsigned long long *__restrict__ prof) {
+               float inv_sinphi, float *__restrict__ out) {
     extern __shared__ __align__(128) unsigned char ut_smem[];
     u64 *full = reinterpret_cast<u64 *>(ut_smem);                 // [kUtMaxSlots] samples landed
     u64 *empty = full + kUtMaxSlots;                               // slot may be refilled (both warps done)
@@ -293,9 +254,7 @@ k_polyphase_ut(const __grid_constant__ UtParams<MAXV> prm, const float *__restri
             float *dst = slots + static_cast<size_t>(s) * g.slot_stride;
             const long long x_lo = static_cast<long long>((b0 + n) * RB * m) - g.back;   // sample staged at dst[0]
             const long long x_hi = x_lo + g.slot_floats;
-            if (g.debug == 2) {                                    // timing experiment: no loads at all
-                if (lane == 0) mbar_arrive(full + s);
-            } else if (x_lo >= 0 && static_cast<u64>(x_hi) <= len) {
+            if (x_lo >= 0 && static_cast<u64>(x_hi) <= len) {
                 if (lane == 0) {
                     mbar_expect_tx(full + s, g.slot_floats * 4);
                     tma_bulk_g2s(dst, signal + x_lo, g.slot_floats * 4, full + s);
@@ -326,14 +285,6 @@ k_polyphase_ut(const __grid_constant__ UtParams<MAXV> prm, const float *__restri
     if (warp > g.warps) return;
 
     // ===== compute warps: tickets are (block, role) pairs; two warps share a block =====
-    // per-phase cycle counters of CTA 0 / warp 0: compiled in with -DAPTB200_UT_PROFILE only (APTB200_TILE_PROFILE=1 prints them)
-#ifdef APTB200_UT_PROFILE
-    const bool profiling = prof != nullptr && blockIdx.x == 0 && warp == 0 && lane == 0;
-    long long pt = profiling ? clock64() : 0;
-#else
-    const bool profiling = false;
-    long long pt = 0;
-#endif
     for (;;) {
         u32 t = 0;
         if (lane == 0) t = atomicAdd(ticket, 1u);
@@ -342,26 +293,17 @@ k_polyphase_ut(const __grid_constant__ UtParams<MAXV> prm, const float *__restri
         if (n >= nblk) break;
         const u32 s = n % g.nslot, parity = (n / g.nslot) & 1;
         float *slot = slots + static_cast<size_t>(s) * g.slot_stride;
-#ifdef APTB200_UT_PROFILE
-        if (profiling) { const long long now_ = clock64(); prof[0] += now_ - pt; pt = now_; }
-#endif
         mbar_wait(full + s, parity);
-#ifdef APTB200_UT_PROFILE
-        if (profiling) { const long long now_ = clock64(); prof[1] += now_ - pt; pt = now_; }
-#endif
         const u64 k0 = (b0 + n) * RB * L;                          // first output of the block
         if (role == 0)
             ut_role<L, 0, NPA, false, Q, VEC, MAXV, ENVELOPE>(prm, g, 0, slot, xch + s, staged + s, parity, role, halo_taps, k0, nout,
-                                                              cosphi2, inv_sinphi, out, lane, profiling, prof, pt);
+                                                              cosphi2, inv_sinphi, out, lane);
         else
             ut_role<L, NPA, NPB, true, Q, VEC, MAXV, ENVELOPE>(prm, g, static_cast<int>(g.stream_b), slot, xch + s, staged + s, parity,
-                                                               role, halo_taps, k0, nout, cosphi2, inv_sinphi, out, lane, profiling, prof, pt);
+                                                               role, halo_taps, k0, nout, cosphi2, inv_sinphi, out, lane);
         fence_proxy_async();                                       // generic writes before the next bulk copy into the slot
         __syncwarp();
         if (lane == 0) mbar_arrive(empty + s);
-#ifdef APTB200_UT_PROFILE
-        if (profiling) { const long long now_ = clock64(); prof[5] += now_ - pt; pt = now_; prof[6] += 1; }
-#endif
     }
 }
 

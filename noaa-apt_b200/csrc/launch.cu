@@ -3,10 +3,8 @@
 
 #include <algorithm>
 #include <atomic>
-#include <cstdio>
 #include <cstdlib>
 #include <cstring>
-#include <type_traits>
 
 #include "aptb200.h"
 #include "common.hpp"
@@ -70,37 +68,18 @@ int launch_polyphase_tiled(const LaunchCtx &c, const float *signal, u64 len, con
     if (tile_begin >= ntiles) return APT_OK;
     const unsigned grid = static_cast<unsigned>(std::min<u64>(ntiles - tile_begin, static_cast<u64>(c.sm_count)));
     const unsigned block = 32 * (tp.groups + kWsEpilogueWarps + 1);   // compute + epilogue + producer warps
-    unsigned long long *prof = nullptr;
-    if (getenv("APTB200_TILE_PROFILE")) {
-        APT_CUDA(cudaMalloc(&prof, 512 * sizeof(unsigned long long)));
-        APT_CUDA(cudaMemsetAsync(prof, 0, 512 * sizeof(unsigned long long), c.stream));
-    }
     if (envelope) {
         auto kern = k_polyphase_ws<true>;
         APT_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(tp.smem_bytes)));
         kern<<<grid, block, tp.smem_bytes, c.stream>>>(signal, len, tile_taps, group_xs, tp, nout, tile_begin, ntiles,
-                                                        cosphi2, sinphi, out, prof);
+                                                        cosphi2, sinphi, out);
     } else {
         auto kern = k_polyphase_ws<false>;
         APT_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(tp.smem_bytes)));
         kern<<<grid, block, tp.smem_bytes, c.stream>>>(signal, len, tile_taps, group_xs, tp, nout, tile_begin, ntiles,
-                                                        cosphi2, sinphi, out, prof);
+                                                        cosphi2, sinphi, out);
     }
     APT_CUDA(cudaGetLastError());
-    if (prof) {
-        unsigned long long h[512];
-        APT_CUDA(cudaStreamSynchronize(c.stream));
-        APT_CUDA(cudaMemcpy(h, prof, sizeof(h), cudaMemcpyDeviceToHost));
-        cudaFree(prof);
-        fprintf(stderr, "[tile profile, CTA 0, %llu tiles, cycles] producer: wait_empty %llu issue %llu | compute warp 0: wait_full %llu "
-                        "main %llu wait_planes %llu write_planes %llu | epilogue warp 0: wait_full %llu work %llu\n",
-                h[8], h[0], h[1], h[2], h[3], h[4], h[5], h[6], h[7]);
-        unsigned long long mn = ~0ull, mx = 0, sum = 0;
-        for (unsigned b = 0; b < grid; ++b) { mn = std::min(mn, h[16 + 2 * b]); mx = std::max(mx, h[16 + 2 * b]); sum += h[16 + 2 * b]; }
-        fprintf(stderr, "[tile profile] per-CTA kernel-body cycles: min %llu avg %llu max %llu; first 12:", mn, sum / grid, mx);
-        for (unsigned b = 0; b < 12 && b < grid; ++b) fprintf(stderr, " %llu(sm%llu)", h[16 + 2 * b], h[17 + 2 * b]);
-        fprintf(stderr, "\n");
-    }
     return APT_OK;
 }
 
@@ -116,27 +95,13 @@ int launch_ut_inst(const LaunchCtx &c, const float *signal, u64 len, const float
         prm.cs[p] = up.cs[p];
         prm.ce[p] = up.ce[p];
     }
-    const UtGeom g{up.l, up.m, up.back, up.slot_floats, up.nslot, up.warps, up.halo_u0, up.halo_n, up.header_bytes, up.slot_stride, up.stream_b, up.debug};
+    const UtGeom g{up.l, up.m, up.back, up.slot_floats, up.nslot, up.warps, up.halo_u0, up.halo_n, up.header_bytes, up.slot_stride, up.stream_b};
     auto kern = k_polyphase_ut<static_cast<int>(kUtL), Q, VEC, MAXV, ENV>;
     APT_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(up.smem_bytes)));
     const unsigned grid = static_cast<unsigned>(std::min<u64>(blk_end - blk_begin, static_cast<u64>(c.sm_count)));
-    unsigned long long *prof = nullptr;
-    if (getenv("APTB200_TILE_PROFILE")) {
-        APT_CUDA(cudaMalloc(&prof, 16 * sizeof(unsigned long long)));
-        APT_CUDA(cudaMemsetAsync(prof, 0, 16 * sizeof(unsigned long long), c.stream));
-    }
     kern<<<grid, 32 * (up.warps + 1), up.smem_bytes, c.stream>>>(prm, signal, len, h, g, nout, blk_begin, blk_end, cosphi2,
-                                                                 1.0f / sinphi, out, prof);
+                                                                 1.0f / sinphi, out);
     APT_CUDA(cudaGetLastError());
-    if (prof) {
-        unsigned long long hp[16];
-        APT_CUDA(cudaStreamSynchronize(c.stream));
-        APT_CUDA(cudaMemcpy(hp, prof, sizeof(hp), cudaMemcpyDeviceToHost));
-        cudaFree(prof);
-        fprintf(stderr, "[ut profile, CTA 0 warp 0: %llu (block, role) units, cycles] ticket %llu wait_full %llu main %llu halo+publish %llu exchange+envelope+stage %llu "
-                        "store+release %llu | plan: q %u warps %u slots %u slot_floats %u chunks %u nvec %u\n",
-                hp[6], hp[0], hp[1], hp[2], hp[3], hp[4], hp[5], up.q, up.warps, up.nslot, up.slot_floats, up.chunks, up.nvec);
-    }
     return APT_OK;
 }
 template <int Q, int VEC, bool ENV>
@@ -167,9 +132,6 @@ int launch_polyphase_ut(const LaunchCtx &c, const float *signal, u64 len, const 
     if (blk_begin >= nblk) return APT_OK;
     if ((reinterpret_cast<uintptr_t>(signal) & 15) || (reinterpret_cast<uintptr_t>(out) & 15) || stream.size() != 4ull * up.nvec)
         return fail(APT_ERR_BAD_ARG, "uniform-tap resampler: misaligned buffers or inconsistent plan");
-    if (up.q == 4)
-        return envelope ? launch_ut_vec<4, true>(c, signal, len, h, up, stream, nout, blk_begin, nblk, cosphi2, sinphi, out)
-                        : launch_ut_vec<4, false>(c, signal, len, h, up, stream, nout, blk_begin, nblk, cosphi2, sinphi, out);
     if (up.q == 2)
         return envelope ? launch_ut_vec<2, true>(c, signal, len, h, up, stream, nout, blk_begin, nblk, cosphi2, sinphi, out)
                         : launch_ut_vec<2, false>(c, signal, len, h, up, stream, nout, blk_begin, nblk, cosphi2, sinphi, out);
@@ -238,13 +200,7 @@ int launch_corr(const LaunchCtx &c, const float *f, u64 ncorr, const int8_t *gua
     return APT_OK;
 }
 
-bool lowpass_corr_supported(u32 ntaps, u32 pw) {
-    return (ntaps == 37 && pw == 3) || (ntaps == 43 && pw == 4) || (ntaps == 61 && pw == 5);
-}
-
-int launch_lowpass_corr(const LaunchCtx &c, const float *e, u64 n, const float *taps_host, u32 ntaps, u32 pw, float *f,
-                        float *corr) {
-    if (n == 0) return APT_OK;
+static LpTaps make_lp_taps(const float *taps_host, u32 ntaps, int dec = 0) {
     LpTaps t{};
     auto tap = [&](long long j) { return j >= 0 && j < static_cast<long long>(ntaps) ? taps_host[j] : 0.f; };
     for (int i = 0; i < 32; ++i) {
@@ -252,6 +208,18 @@ int launch_lowpass_corr(const LaunchCtx &c, const float *e, u64 n, const float *
         t.a_odd[i] = make_float2(tap(2 * i + 1), tap(2 * i));
     }
     for (int j = -1; j < 63; ++j) t.p[j + 1] = make_float2(tap(j), tap(j + 1));
+    for (int j = -dec; j < 72 - dec; ++j) t.pd[j + dec] = make_float2(tap(j), tap(j + dec));
+    return t;
+}
+
+bool lowpass_corr_supported(u32 ntaps, u32 pw) {
+    return (ntaps == 37 && pw == 3) || (ntaps == 43 && pw == 4) || (ntaps == 61 && pw == 5);
+}
+
+int launch_lowpass_corr(const LaunchCtx &c, const float *e, u64 n, const float *taps_host, u32 ntaps, u32 pw, float *f,
+                        float *corr) {
+    if (n == 0) return APT_OK;
+    const LpTaps t = make_lp_taps(taps_host, ntaps);
     const u64 ncorr = n > 38ull * pw ? n - 38ull * pw : 0;
     const u64 ntiles = (n + kLpTile - 1) / kLpTile;
     // persistent: exactly the resident CTAs, each walks its tiles with the next tile's loads in flight
@@ -305,34 +273,17 @@ int launch_pick(const LaunchCtx &c, u64 ncorr, u64 nwork, u32 row, u32 dist, con
     int dummy = 0;
     int &nk = kernels_launched ? *kernels_launched : dummy;
     nk = 1;
-    // Which parallel orbit walk: APTB200_PICK = compress | cluster | grid forces one; by default the whole-GPU cooperative
-    // walk (39 us, but it needs every SM) when the device is otherwise idle, the 8-CTA cluster walk (60 us on 8 SMs) when
-    // other recordings are in flight on other streams (batch: 338 k vs 280 k Msamples/s at 64 streams).
+    // Which parallel orbit walk: APTB200_PICK = cluster | grid forces one; by default the whole-GPU cooperative walk (39 us,
+    // but it needs every SM) when the device is otherwise idle, the 8-CTA cluster walk (60 us on 8 SMs) when other
+    // recordings are in flight on other streams (batch: 338 k vs 280 k Msamples/s at 64 streams).
     static const int forced = [] {
         const char *e = getenv("APTB200_PICK");
-        if (getenv("APTB200_GRID_PICK")) return 2;
         if (!e) return -1;
-        return !strcmp(e, "compress") ? 0 : !strcmp(e, "cluster") ? 1 : !strcmp(e, "grid") ? 2 : -1;
+        return !strcmp(e, "cluster") ? 1 : !strcmp(e, "grid") ? 2 : -1;
     }();
     const int mode = forced >= 0 ? forced : (c.busy ? 1 : 2);
     const u64 nr = (ncorr + row - 1) / row;
-    if (scratch && mode == 0 && nr + 1 <= static_cast<u64>(kPickEMax - 2) * kPickR) {
-        // compressed walk: J0 and E = J0^8 over the whole GPU, then one CTA (see kernels_sync.cuh)
-        const size_t smem = (3ull * kPickKMax + kPickEMax) * sizeof(u32);
-        // the attribute belongs to the (function, device) pair: one flag per device, not one per process
-        static std::atomic<signed char> attr_final[kMaxDevices];
-        if (smem_attr_once(attr_final, k_pick_final, smem)) {
-            PickScratch sc = *scratch;
-            const unsigned grid = (sc.cap + 1 + 255) / 256;       // one thread per possible node; the kernels know how many exist
-            k_pick_j0<<<grid, 256, 0, c.stream>>>(ncorr, row, dist, ri, positions, max_positions, result, sc);
-            k_pick_e8<<<grid, 256, 0, c.stream>>>(ncorr, row, ri, max_positions, result, sc);
-            k_pick_final<<<1, 1024, smem, c.stream>>>(ncorr, nwork, row, dist, ri, positions, max_positions, result, sc);
-            APT_CUDA(cudaGetLastError());
-            nk = 3;
-            return APT_OK;
-        }
-    }
-    if (scratch && mode <= 1 && nr <= 20000) {
+    if (scratch && mode == 1 && nr <= 20000) {
         // one 8-CTA cluster, jump tables in distributed shared memory (larger recordings: the whole-GPU cooperative grid)
         const size_t smem = 2ull * kPickClusterPer * sizeof(u32);
         static std::atomic<signed char> attr_cluster[kMaxDevices];
@@ -375,72 +326,28 @@ int launch_pick(const LaunchCtx &c, u64 ncorr, u64 nwork, u32 row, u32 dist, con
     return APT_OK;
 }
 
-static LpTaps make_lp_taps(const float *taps_host, u32 ntaps, int dec = 0) {
-    LpTaps t{};
-    auto tap = [&](long long j) { return j >= 0 && j < static_cast<long long>(ntaps) ? taps_host[j] : 0.f; };
-    for (int i = 0; i < 32; ++i) {
-        t.a_even[i] = make_float2(tap(2 * i), tap(2 * i - 1));
-        t.a_odd[i] = make_float2(tap(2 * i + 1), tap(2 * i));
-    }
-    for (int j = -1; j < 63; ++j) t.p[j + 1] = make_float2(tap(j), tap(j + 1));
-    for (int j = -dec; j < 72 - dec; ++j) t.pd[j + dec] = make_float2(tap(j), tap(j + dec));
-    return t;
-}
-
-// Rows of 32 low-passed samples per tile of the record kernel (64, or 32 with APTB200_REC_TB=32); fixed per process.
-static int records_tb() {
-    static const int tb = [] {
-        const char *e = getenv("APTB200_REC_TB");
-        return e && atoi(e) == 32 ? 32 : 64;
-    }();
-    return tb;
-}
-
-u32 records_tile(u32 pw) { return static_cast<u32>(rec_tile_outputs(static_cast<int>(pw), records_tb())); }
+u32 records_tile(u32 pw) { return static_cast<u32>(rec_tile_outputs(static_cast<int>(pw))); }
 
 int launch_lowpass_records(const LaunchCtx &c, const float *e, u64 n, u64 ncorr, const float *taps_host, u32 ntaps, u32 pw,
                            SyncCtl *ctl, TileDesc *desc, Rec *pool, u32 pool_cap, u32 region, u32 ntiles) {
     if (ntiles == 0) return APT_OK;
     const LpTaps t = make_lp_taps(taps_host, ntaps);
-    const int tb = records_tb();
-    static const int nbuf = [] {
-        const char *e = getenv("APTB200_REC_NBUF");
-        return e && atoi(e) == 2 ? 2 : 1;
-    }();
-    auto launch = [&](auto kern, auto nwc) {
-        constexpr int NWc = decltype(nwc)::value;
-        const size_t smem = static_cast<size_t>(nbuf) * NWc * rec_smem_floats(tb) * sizeof(float);
-        if (smem > (48u << 10))      // the attribute is per device: set on every launch, not cached
-            cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
+    // one warp per CTA, as many CTAs as are resident; 9.4 KB of shared memory each needs no opt-in
+    constexpr size_t smem = kRecSmemFloats * sizeof(float);
+    static_assert(smem <= (48u << 10), "record kernel: dynamic shared memory above the default limit");
+    auto launch = [&](auto kern) {
         static const int per_sm = [&] {
             int v = 0;
-            if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&v, kern, 32 * NWc, smem) != cudaSuccess || v < 1) v = 1;
+            if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&v, kern, 32, smem) != cudaSuccess || v < 1) v = 1;
             return v;
         }();
-        const unsigned want = (ntiles + NWc - 1) / NWc;
-        unsigned ctas = static_cast<unsigned>(per_sm);
-        static const int forced_w = [] { const char *e = getenv("APTB200_REC_WARPS"); return e ? atoi(e) : 0; }();
-        if (forced_w > 0) ctas = std::max(1u, std::min<unsigned>(static_cast<unsigned>(forced_w) / NWc, ctas));
-        const unsigned grid = std::min<unsigned>(want, static_cast<unsigned>(c.sm_count) * ctas);
-        kern<<<grid, 32 * NWc, smem, c.stream>>>(e, n, ncorr, t, ctl, desc, pool, pool_cap, region, ntiles);
+        const unsigned grid = std::min<unsigned>(ntiles, static_cast<unsigned>(c.sm_count) * per_sm);
+        kern<<<grid, 32, smem, c.stream>>>(e, n, ncorr, t, ctl, desc, pool, pool_cap, region, ntiles);
     };
-    using I1 = std::integral_constant<int, 1>;
-    using I2 = std::integral_constant<int, 2>;
-    auto pick = [&](auto tbc, auto nbc) -> int {
-        constexpr int TBc = decltype(tbc)::value, NBc = decltype(nbc)::value;
-        if (ntaps == 37 && pw == 3) {
-            launch(k_lowpass_records<37, 3, TBc, NBc>, I1{});
-        } else if (ntaps == 43 && pw == 4) launch(k_lowpass_records<43, 4, TBc, NBc>, I1{});
-        else if (ntaps == 61 && pw == 5) launch(k_lowpass_records<61, 5, TBc, NBc>, I1{});
-        else return fail(APT_ERR_BAD_ARG, "no fused low-pass/record kernel for %u taps, pixel width %u", ntaps, pw);
-        return APT_OK;
-    };
-    using T32 = std::integral_constant<int, 32>;
-    using T64 = std::integral_constant<int, 64>;
-    int rc;
-    if (tb == 64) rc = nbuf == 2 ? pick(T64{}, I2{}) : pick(T64{}, I1{});
-    else rc = nbuf == 2 ? pick(T32{}, I2{}) : pick(T32{}, I1{});
-    if (rc != APT_OK) return rc;
+    if (ntaps == 37 && pw == 3) launch(k_lowpass_records<37, 3>);
+    else if (ntaps == 43 && pw == 4) launch(k_lowpass_records<43, 4>);
+    else if (ntaps == 61 && pw == 5) launch(k_lowpass_records<61, 5>);
+    else return fail(APT_ERR_BAD_ARG, "no fused low-pass/record kernel for %u taps, pixel width %u", ntaps, pw);
     APT_CUDA(cudaGetLastError());
     return APT_OK;
 }
@@ -517,7 +424,7 @@ int launch_quantize_i16(const LaunchCtx &c, const float *x, u64 n, PostCtl *ctl,
 static size_t align_up(size_t v) { return (v + 255) & ~static_cast<size_t>(255); }
 
 size_t pick_scratch_bytes(u32 max_blocks, u32 max_positions, u32 cap) {
-    return align_up((static_cast<size_t>(max_blocks) + 1) * 4) + 5 * align_up((static_cast<size_t>(cap) + 1) * 4) +
+    return align_up((static_cast<size_t>(max_blocks) + 1) * 4) + 4 * align_up((static_cast<size_t>(cap) + 1) * 4) +
            align_up((static_cast<size_t>(max_positions) + 1) * 4) + align_up(8);
 }
 
@@ -534,7 +441,6 @@ PickScratch pick_scratch_carve(void *base, u32 max_blocks, u32 max_positions, u3
     s.cand_peak = take(static_cast<size_t>(cap) + 1);
     s.ja = take(static_cast<size_t>(cap) + 1);
     s.jb = take(static_cast<size_t>(cap) + 1);
-    s.idx = take(static_cast<size_t>(cap) + 1);
     s.orbit = take(static_cast<size_t>(max_positions) + 1);
     s.ticket = take(2);
     s.cap = cap;

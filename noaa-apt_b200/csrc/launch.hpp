@@ -29,7 +29,7 @@ constexpr u32 kSyncRedo = 100;
 
 // Control block of the fused sync stage (kernels_sync2.cuh); zeroed at the start of every job.
 struct SyncCtl {
-    u32 tile_ticket;   // (unused since the tiles of k_lowpass_records are dealt out statically)
+    u32 pad0;          // keeps the layout; pad[0] below is the picker's ticket
     u32 pool_cursor;   // record-pool entries handed out
     u32 overflow;      // the pool was exhausted
     u32 root_cursor;   // dense root ids handed out by k_resolve_roots (= number of roots when it is done)
@@ -72,8 +72,7 @@ struct PickScratch {
     u32 *block_off;    // [nblocks + 1] exclusive scan of root_count (dense root numbering)
     u32 *cand_s;       // [cap + 1] start position of each candidate
     u32 *cand_peak;    // [cap + 1] firstroot(start)
-    u32 *ja, *jb;      // [cap + 1] jump tables (J0, and the global ping-pong pair when smem is too small / E = J0^8)
-    u32 *idx;          // [cap + 1] compressed walk: image flag, then compact id of a node
+    u32 *ja, *jb;      // [cap + 1] jump tables (J0, and the global ping-pong pair when smem is too small)
     u32 *orbit;        // [max_positions + 1]
     u32 *ticket;       // [2] last-CTA tickets of k_roots / k_pick_links (zero between launches)
     u32 cap;           // candidate capacity
@@ -102,7 +101,6 @@ struct TilePlan {
     u32 smem_bytes;    // dynamic shared memory
     u32 ctas_per_sm;   // 2 when two CTAs fit an SM, else 1
     u64 off2;          // 2*((N-1)/2)
-    u32 debug;         // 0 normal; 1 skip the FMA loop; 2 skip the loads (timing experiments only)
 };
 
 // Geometry of the uniform-tap kernel (kernels_ut.cuh) for one (L, M, taps) triple; built by make_ut_plan.
@@ -115,7 +113,7 @@ constexpr u32 kUtChunk = 8;            // samples per loop iteration (chunk) of 
 struct UtPlan {
     u32 l, m;
     u32 np;            // pairs of outputs per row = ceil(L/2)
-    u32 q;             // rows per thread (4, or 2 / 1 when the rows are long: 96 / 192 kHz input)
+    u32 q;             // rows per thread: 2, or 1 when two rows do not fit shared memory (192 kHz input)
     u32 rb;            // rows per block = 32*q; a block = rb*L outputs from one contiguous span of the signal
     u32 vec;           // 4/2/1: widest aligned shared-memory load of a row's samples (M % 4 == 0 / M % 2 == 0 / odd)
     u32 back;          // samples staged in front of a block's first row (window of output k0-1), multiple of 4
@@ -130,7 +128,6 @@ struct UtPlan {
     u32 halo_u0, halo_n;   // output L-1: first sample relative to its row, number of taps
     u32 cs[8], ce[8];  // pair p is active in chunks [cs[p], ce[p])
     u64 off2;
-    u32 debug;
 };
 
 // Geometry of the phase-major resampler (kernels_ph.cuh) for large interpolation factors; built by make_ph_plan.

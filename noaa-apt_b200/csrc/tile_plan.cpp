@@ -1,6 +1,5 @@
 // Host-side geometry of the tiled polyphase kernel (kernels_fast.cuh).
 #include <algorithm>
-#include <cstdlib>
 #include <numeric>
 
 #include "launch.hpp"
@@ -161,8 +160,6 @@ static bool try_tile_plan(u32 halves, u32 l, u32 m, const std::vector<float> &ta
     tp.ctas_per_sm = 1;
     tp.stage_floats = static_cast<u32>(stage_floats);
     tp.off2 = off2;
-    tp.debug = 0;
-    if (const char *e = getenv("APTB200_TILE_DEBUG")) tp.debug = static_cast<u32>(atoi(e));
     return true;
 }
 

@@ -64,33 +64,25 @@ bool make_ut_plan(u32 l, u32 m, const std::vector<float> &taps, UtPlan &up, std:
     const u32 back = (m > halo_u0 ? (m - halo_u0 + 3) / 4 * 4 : 0);
     const u32 header = (1024 + halo_n * 4 + 127) / 128 * 128;
     if (header > 16 * 1024) return false;
-    u32 want_warps = 0, want_spare = 0;                          // experiment knobs
-    if (const char *e = getenv("APTB200_UT_WARPS")) want_warps = static_cast<u32>(atoi(e));
-    if (const char *e = getenv("APTB200_UT_SPARE")) want_spare = static_cast<u32>(atoi(e));
     bool ok = false;
-    u32 want_q = 0;
-    if (const char *e = getenv("APTB200_UT_Q")) want_q = static_cast<u32>(atoi(e));
     // rows per thread: 2 measured best (48 kHz: 71 us against 76 for q = 4, which leaves room for only 12 warps;
     // 96 kHz: 142 us against 181 for q = 1, whose one uniform load per FFMA2 saturates the uniform-load port);
-    // q = 1 only when two rows per thread do not fit shared memory (192 kHz); q = 4 on request (APTB200_UT_Q)
-    for (u32 q : {2u, 1u, 4u}) {
-        if (want_q ? q != want_q : q == 4) continue;
+    // q = 1 only when two rows per thread do not fit shared memory (192 kHz)
+    for (u32 q : {2u, 1u}) {
         const u32 rb = 32 * q;
         const u64 slot_floats = (static_cast<u64>(back) + static_cast<u64>(rb - 1) * m + static_cast<u64>(kUtChunk) * chunks + 3) / 4 * 4;
         const u64 slot_stride = slot_floats + 2 * rb + 4;          // + the exchange words of the two roles
         const u64 slot_bytes = slot_stride * 4;
         if (static_cast<u64>(rb) * l > slot_floats) continue;      // the block's outputs are transposed through its slot
         const u32 nslot = static_cast<u32>(std::min<u64>(kUtMaxSlots, (kSmemBudget - header) / slot_bytes));
-        u32 spare = static_cast<u32>(std::max<u64>(2, (kInflightBytes + slot_bytes - 1) / slot_bytes));
-        if (want_spare) spare = want_spare;
+        const u32 spare = static_cast<u32>(std::max<u64>(2, (kInflightBytes + slot_bytes - 1) / slot_bytes));
         if (nslot < spare + 3) continue;                           // at least 3 blocks (6 warps) in compute
-        u32 warps = std::min<u32>(q >= 4 ? 14 : 24, 2 * (nslot - spare));   // two warps per block in compute
-        if (want_warps && want_warps <= warps) warps = want_warps & ~1u;
+        const u32 warps = std::min<u32>(24, 2 * (nslot - spare));   // two warps per block in compute
         up.q = q;
         up.rb = rb;
         up.slot_floats = static_cast<u32>(slot_floats);
         up.warps = warps;
-        up.nslot = std::min(nslot, warps / 2 + spare + (want_spare ? 0 : 1));
+        up.nslot = std::min(nslot, warps / 2 + spare + 1);
         up.slot_stride = static_cast<u32>(slot_stride);
         up.header_bytes = header;
         up.smem_bytes = header + up.nslot * static_cast<u32>(slot_bytes);
@@ -113,8 +105,6 @@ bool make_ut_plan(u32 l, u32 m, const std::vector<float> &taps, UtPlan &up, std:
         up.cs[p] = cs[p];
         up.ce[p] = ce[p];
     }
-    up.debug = 0;
-    if (const char *e = getenv("APTB200_TILE_DEBUG")) up.debug = static_cast<u32>(atoi(e));
     return true;
 }
 

@@ -1,5 +1,6 @@
 """Times the resample+envelope kernel alone (decoder profiling events) on a device-resident synthetic recording.
-Timing experiments only (APTB200_TILE_DEBUG modes produce garbage output on purpose)."""
+RATE, SECS and ITERS set the input; APTB200_NO_UNIFORM_TAPS=1 times the tiled kernel (k_polyphase_ws) instead of the
+uniform-tap one."""
 import os, sys, ctypes as C
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
@@ -16,11 +17,8 @@ out = torch.empty(dec.out_bound(x.size), dtype=torch.float32, device="cuda")
 dec.set_profiling(True)
 times = []
 for it in range(int(os.environ.get("ITERS", "12"))):
-    try:
-        dec.submit_device(dx.data_ptr(), 0, x.size, True, out.data_ptr(), out.numel())
-        dec.wait()
-    except Exception as e:  # debug modes break the sync search; the kernel times are still valid
-        pass
+    dec.submit_device(dx.data_ptr(), 0, x.size, True, out.data_ptr(), out.numel())
+    dec.wait()
     t = dict(dec.kernel_times_ms())
     times.append(t.get("resample_envelope", float("nan")))
 print("resample_envelope ms: median %.4f  min %.4f  (n=%d)" % (float(np.median(times[2:])), min(times[2:]), len(times) - 2))
